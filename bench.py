@@ -32,6 +32,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the modules imported from the tree leave nothing in it (it may be read-only)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -212,7 +213,7 @@ def run_reference(args, rank):
         for _ in range(max(1, min(args.warmup, 2))):
             pool.map(_cpu_frames, [(i, per) for i in range(cores)])
         t0 = time.perf_counter()
-        steps = max(1, min(args.steps, 20))   # keep the whole run within minutes
+        steps = args.steps
         for _ in range(steps):
             pool.map(_cpu_frames, [(i, per) for i in range(cores)])
         dt = time.perf_counter() - t0
@@ -231,31 +232,19 @@ def run_reference(args, rank):
 
 
 # --------------------------------------------------------------------------- GPU arm
-MIN_REGION_S = 0.06          # timed regions shorter than this are repeated (median reported) until >= 0.05 s have been timed in all
-
-
-def timed_region(step, steps, barrier, torch, first_index=0, allmax=None):
-    """CUDA-event time of exactly `steps` calls of step(i), barrier + synchronize on both sides.  When the region is
-    shorter than MIN_REGION_S it is repeated (same K steps each time) and the MEDIAN is returned, so that a 20-step
-    run of a 0.1 ms step is not a 2 ms sample.  Returns (ms of one K-step region, repeats, total timed seconds)."""
-    def once():
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        barrier()
-        e0.record()
-        for i in range(steps):
-            step(first_index + i)
-        e1.record()
-        barrier()
-        return e0.elapsed_time(e1)
-    first = once()
-    # every rank must repeat the region the SAME number of times (each repetition contains barriers): the count is
-    # decided on the slowest rank's first measurement, never on the local one (a rank-local count deadlocks at N > 1)
-    ref = allmax(first) if allmax is not None else first
-    reps = 1
-    if ref * 1e-3 < MIN_REGION_S:
-        reps = int(min(400, max(3, np.ceil(MIN_REGION_S / max(ref * 1e-3, 1e-6)) + 1))) | 1      # odd
-    times = [first] + [once() for _ in range(reps - 1)]
-    return float(np.median(times)), reps, float(np.sum(times)) * 1e-3
+def timed_region(step, steps, barrier, torch, first_index=0):
+    """CUDA-event time in ms of exactly `steps` calls of step(i), barrier + synchronize on both sides: --steps is the
+    number of steps every timed region runs, whatever its length."""
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    e1.record()                     # an event is created by its first record: keep that out of the timed window
+    barrier()
+    e0.record()
+    for i in range(steps):
+        step(first_index + i)
+    e1.record()
+    barrier()
+    return e0.elapsed_time(e1)
 
 
 def numa_bind(local_rank, torch):
@@ -358,18 +347,23 @@ def run_gpu(args, rank, local_rank, world):
         r.execute(batches[i % N_BANKS], out=spec_out)
 
     # ---- device-resident throughput ("value")
-    for i in range(args.warmup):
-        step(i)
-    barrier()
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
         time.sleep(0.25)
+    for i in range(args.warmup):
+        step(i)
+    barrier()
     launches0 = r.ctx.launch_count
     t_wall0 = time.time()
-    ms, reps, region_s = timed_region(step, args.steps, barrier, torch, allmax=allmax)
+    ms = timed_region(step, args.steps, barrier, torch)
     t_wall1 = time.time()
-    launches = (r.ctx.launch_count - launches0) // reps
+    launches = r.ctx.launch_count - launches0
+    if args.dump_outputs:
+        # what the caller of the timed path received from its last step: the spectrogram batch of that step
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        name = "spectrogram" if world == 1 else f"spectrogram_rank{rank}"
+        np.save(os.path.join(args.dump_outputs, name + ".npy"), spec_out.cpu().numpy())
     # a long enough region for the clock sampler: keep the GPU under the same load for >= 1.5 s
     clocks = None
     if sampler:
@@ -405,7 +399,7 @@ def run_gpu(args, rank, local_rank, world):
         try:
             for i in range(max(3, args.warmup // 2)):
                 gstep(i)
-            gms, greps, _ = timed_region(gstep, args.steps, barrier, torch, allmax=allmax)
+            gms = timed_region(gstep, args.steps, barrier, torch)
             gms = allmax(gms)
             # every rank must now hold every rank's rows: compare a checksum of the gathered batch across ranks,
             # and this rank's own rows with what it rendered without the collective
@@ -440,7 +434,7 @@ def run_gpu(args, rank, local_rank, world):
     hs.set_requests(sid, silent=sil)
     for _ in range(max(3, args.warmup // 4)):
         hs.run()
-    e2e_ms, _, _ = timed_region(lambda i: hs.run(), args.steps, barrier, torch, allmax=allmax)
+    e2e_ms = timed_region(lambda i: hs.run(), args.steps, barrier, torch)
     e2e_ms_max = allmax(e2e_ms)
     checksum = float(hs.h_spec.double().sum())
     hs_bytes = (hs.h2d_bytes, hs.d2h_bytes)
@@ -494,7 +488,7 @@ def run_gpu(args, rank, local_rank, world):
     try:
         if miss_info is not None:
             raise RuntimeError(miss_info["error"])
-        mms, _, _ = timed_region(mstep, args.steps, mbarrier, torch, allmax=allmax)
+        mms = timed_region(mstep, args.steps, mbarrier, torch)
         mms = allmax(mms)
         miss_info = {"value": B * world * args.steps / (mms * 1e-3), "unit": UNIT, "ms_per_step": mms / args.steps,
                      "miss_rate": n_miss / B, "h2d_bytes_per_step": int(n_miss * TAPS * 8),
@@ -528,8 +522,8 @@ def run_gpu(args, rank, local_rank, world):
     try:
         if not ok_api:
             raise RuntimeError(err or "set-up failed on another rank")
-        ams, _, _ = timed_region(api_step, args.steps, barrier, torch, allmax=allmax)
-        bms, _, _ = timed_region(arr_step, args.steps, barrier, torch, allmax=allmax)
+        ams = timed_region(api_step, args.steps, barrier, torch)
+        bms = timed_region(arr_step, args.steps, barrier, torch)
         api_info = {"api_path": {"value": B * world * args.steps / (allmax(ams) * 1e-3), "unit": UNIT,
                                  "what": "execute(prepare(list[AudioRequest])) every step: request resolution + H2D of the request array + launches"},
                     "api_path_arrays": {"value": B * world * args.steps / (allmax(bms) * 1e-3), "unit": UNIT,
@@ -554,7 +548,7 @@ def run_gpu(args, rank, local_rank, world):
                 r2.execute(b2[i % N_BANKS], out=out2)
             for i in range(args.warmup):
                 step2(i)
-            ms2, reps2, _ = timed_region(step2, args.steps, barrier, torch)
+            ms2 = timed_region(step2, args.steps, barrier, torch)
             r2.ctx.set_kernel_timing(True)
             for i in range(args.steps):
                 step2(i)
@@ -563,7 +557,7 @@ def run_gpu(args, rank, local_rank, world):
             step(0); step2(0)
             torch.cuda.synchronize()
             live2 = read_live_step(other)
-            alt = {"plan": other, "value": B * args.steps / (ms2 * 1e-3), "unit": UNIT, "ms_per_step": ms2 / args.steps, "repeats": reps2,
+            alt = {"plan": other, "value": B * args.steps / (ms2 * 1e-3), "unit": UNIT, "ms_per_step": ms2 / args.steps,
                    "kernel_ms_all": {k: v[0] / args.steps for k, v in kt2.items() if v[1]},
                    "traffic": live2["dram_bytes"] if live2 else None, "traffic_source": live2["source"] if live2 else None,
                    "traffic_over_algorithmic": (live2["dram_bytes"] / (ALG_BYTES_PER_FRAME * B)) if live2 else None,
@@ -618,8 +612,7 @@ def run_gpu(args, rank, local_rank, world):
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": step_ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "config": cfg,
-            "timed_region_s": region_s, "timed_region_repeats": reps,
-            "timed_region_note": f"the K={args.steps}-step region was timed {reps} time(s); ms_per_step is the median region / K",
+            "timed_region_s": ms_max * 1e-3,
             "roofline": {
                 "bound": "hbm", "kernel": dom, "achieved": achieved, "peak": peak, "unit": "GB/s",
                 "frac": achieved / peak,
@@ -688,7 +681,7 @@ def plugin_path_leg(args, r, bank_host, sid, dev, world, barrier, allmax, agree,
     if not agree(err is None):
         return {"error": err or "set-up failed on another rank"}
     B = ENVS_PER_GPU
-    pms, _, _ = timed_region(pstep, args.steps, barrier, torch, allmax=allmax)
+    pms = timed_region(pstep, args.steps, barrier, torch)
     pms = allmax(pms)
     return {"value": B * world * args.steps / (pms * 1e-3), "unit": UNIT, "ms_per_step": pms / args.steps,
             "what": "per env: SpectrogramSensor.get_observation -> DeferredObservation handle; per step: batch_obs -> ONE render into "
@@ -725,22 +718,22 @@ def _plugin_setup(args, r, bank_host, sid, dev, torch):
 
 
 def extra_workloads(args, dev, torch, barrier):
-    """The other BASELINE.json configs on ONE GPU, inputs resident (same timing rules; short regions are repeated):
+    """The other BASELINE.json configs on ONE GPU, inputs resident (same timing rules, --steps steps each):
     C3 head / valid / log-mel at 512 envs, C4 (ambisonic decode + convolution) at 256 envs, C5 rollout (16 envs)."""
     from soundspaces_b200 import AudioRequest, BatchedAudioRenderer
     from synth import make_source
     peak = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))["hbm_gbs"] if os.path.exists(os.path.join(ROOT, "MEASURED_PEAKS.json")) else 6650.0
     res = {}
-    steps, warm = max(10, min(args.steps, 50)), 5
+    steps, warm = args.steps, 5
     rng = np.random.default_rng(0)
     sr, L, Bc = 16000, 48000, 512
 
     def run(name, fn, frames_per_step, bytes_per_frame, flop_per_frame, note):
         for i in range(warm):
             fn(i)
-        ms, reps, _ = timed_region(fn, steps, barrier, torch)
+        ms = timed_region(fn, steps, barrier, torch)
         v = frames_per_step * steps / (ms * 1e-3)
-        res[name] = {"value": v, "unit": UNIT, "ms_per_step": ms / steps, "envs": frames_per_step, "repeats": reps,
+        res[name] = {"value": v, "unit": UNIT, "ms_per_step": ms / steps, "envs": frames_per_step,
                      "algorithmic_bytes_per_frame": bytes_per_frame, "path_frac_hbm": v * bytes_per_frame / 1e9 / peak,
                      "algorithmic_flop_per_frame": flop_per_frame, "fp32_frac_nominal": v * flop_per_frame / (FP32_PEAK_TFLOPS * 1e12),
                      "workload": note}
@@ -799,17 +792,17 @@ def extra_workloads(args, dev, torch, barrier):
     except Exception as e:          # noqa: BLE001
         res["C4_error"] = repr(e)[:200]
     try:
-        res["C1_single_env"] = c1_single_env(dev, torch)
+        res["C1_single_env"] = c1_single_env(dev, torch, reps=args.steps)
     except Exception as e:          # noqa: BLE001
         res["C1_error"] = repr(e)[:200]
     try:
-        res["C5_rollout"] = c5_rollout(dev, torch)
+        res["C5_rollout"] = c5_rollout(dev, torch, num_steps=args.steps)
     except Exception as e:          # noqa: BLE001
         res["C5_error"] = repr(e)[:200]
     return res
 
 
-def c1_single_env(dev, torch, sr=44100, taps=22050, reps=200):
+def c1_single_env(dev, torch, reps, sr=44100, taps=22050):
     """BASELINE.json configs[0] (SURVEY C1): ONE env, 1-s clip at 44.1 kHz x 22050-tap binaural RIR read from a wav file on
     disk, through the reference's own per-env call: sim.get_current_spectrogram_observation(compute_spectrogram) -> host
     ndarray (compat mode: one render + blocking read-back per call; memo defeated by alternating two receiver nodes whose
@@ -852,7 +845,7 @@ def c1_single_env(dev, torch, sr=44100, taps=22050, reps=200):
                         "(render B=1 + blocking device->host copy per call; RIR resident after the first read)"}
 
 
-def c5_rollout(dev, torch, n_envs=16, num_steps=150, sr=16000, taps=16000):
+def c5_rollout(dev, torch, num_steps, n_envs=16, sr=16000, taps=16000):
     """BASELINE.json configs[4]: DD-PPO rollout, 16 envs per GPU, audio observation fused into the step (trace-replay
     env, SURVEY.md 8(d)): env-steps/s with the env_time / pth_time split of ppo_trainer.py:125-194."""
     from soundspaces_b200.replay import AudioPolicy, ReplayScene, ReplaySim, ReplayVectorEnv, collect_rollout
@@ -905,6 +898,9 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="N = 1: skip the other BASELINE configs (extra_workloads)")
     ap.add_argument("--no-numa", action="store_true", help="N > 1: do not bind ranks to their GPU's NUMA node")
     ap.add_argument("--miss-rate", type=float, default=0.10, help="e2e_resident_bank: fraction of envs whose RIR is uploaded per step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the spectrogram batch the timed path returned in its last step to DIR/spectrogram.npy "
+                         "(float32; one file per rank, spectrogram_rank<r>.npy, when --gpus > 1)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))

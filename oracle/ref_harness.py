@@ -1,13 +1,12 @@
 """Stub-import harness: load the UNMODIFIED reference modules
 ``soundspaces/simulator.py``, ``soundspaces/continuous_simulator.py`` and
-``soundspaces/tasks/nav.py`` from ``/root/reference`` and drive their audio
-methods on synthetic wav trees.
+``soundspaces/tasks/nav.py`` from a sound-spaces checkout (``SOUNDSPACES_REFERENCE``)
+and drive their audio methods on synthetic wav trees.
 
 TEST INFRASTRUCTURE ONLY (see ``oracle/audio_oracle.py``).  Works only where
-the reference tree exists (the build container); the GPU box has no
-``/root/reference`` so nothing that runs there may call :func:`load_reference`.
-Used by ``tests/golden/make_golden.py`` (fixture generation) and by the
-``needs_reference`` CPU tests.
+a reference checkout exists, so only ``tests/golden/make_golden.py`` (fixture
+generation) calls :func:`load_reference`; the tests use the recorded fixtures
+and the plain helpers (``AttrDict``, ``write_rir``, ``make_discrete_sim``).
 
 habitat / habitat_sim / gym / librosa / skimage are absent and un-installable
 here, so they are replaced by inert stubs; ``librosa.stft`` and

@@ -12,26 +12,24 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "needs_reference: needs /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
-    from oracle import ref_harness
-    have_ref = ref_harness.reference_available()
     try:
         import torch
         have_gpu = torch.cuda.is_available()
     except Exception:
         have_gpu = False
     for item in items:
-        if "needs_reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="reference tree not present on this box"))
         if "gpu" in item.keywords and not have_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
 
 
 @pytest.fixture(scope="session")
 def golden():
-    path = os.path.join(ROOT, "tests", "golden", "reference_golden.npz")
-    with np.load(path) as z:
-        return {k: z[k] for k in z.files}
+    """The reference's recorded outputs (tests/golden/make_golden.py): spectrograms and metadata, and the waveforms."""
+    out = {}
+    for name in ("reference_golden.npz", "reference_golden_waves.npz"):
+        with np.load(os.path.join(ROOT, "tests", "golden", name)) as z:
+            out.update({k: z[k] for k in z.files})
+    return out

@@ -1,15 +1,21 @@
-"""Generate tests/golden/reference_golden.npz by running the UNMODIFIED
-reference (``/root/reference/soundspaces/{simulator,continuous_simulator,
-tasks/nav}.py``) through ``oracle/ref_harness.py`` on seeded synthetic wav
-trees.  Run in the build container only:
+"""Generate the reference fixtures under tests/golden/ by running the UNMODIFIED
+reference (``soundspaces/{simulator,continuous_simulator,tasks/nav}.py`` of a
+sound-spaces checkout, located by ``SOUNDSPACES_REFERENCE``) through
+``oracle/ref_harness.py`` on seeded synthetic wav trees:
 
-    python tests/golden/make_golden.py
+    SOUNDSPACES_REFERENCE=<sound-spaces checkout> python tests/golden/make_golden.py
 
-The fixtures hold the reference's own outputs; ``tests/test_oracle_golden.py``
-pins ``oracle/audio_oracle.py`` to them and the GPU parity tests compare the
-CUDA path against the same arrays.
+The fixtures hold the reference's own outputs (``reference_golden.npz``:
+spectrograms and metadata, ``reference_golden_waves.npz``: waveforms,
+``reference_classes.json``: the member names of its simulator classes);
+``tests/test_oracle_golden.py`` pins ``oracle/audio_oracle.py`` to them and the
+GPU parity tests compare the CUDA path against the same arrays.  The tests need
+only these files, never the reference itself.
 """
+import inspect
+import json
 import os
+import re
 import sys
 import tempfile
 
@@ -62,6 +68,16 @@ CONTINUOUS_EDGE_CASES = {
 }
 
 
+# one 3-s clip x 21000-tap RIR at azimuth 180, mp3d layout, rendered at each audio index: the oracle must reproduce the
+# reference bit for bit (tests/test_oracle_golden.py::test_oracle_vs_reference_outputs)
+AUDIO_INDEX_CASE = dict(sr=16000, S=48000, L=21000, seed=77, dataset="mp3d", scene="sc", rotation_angle=180,
+                        receiver=4, source=9, audio_indices=(0, 1, 2))
+
+# the waveforms a test feeds back in as input are stored whole; every other discrete waveform as every 5th sample
+# (the spectrogram of every case is stored whole)
+FULL_WAVES = ("a2_16k/wave",)
+
+
 def discrete_inputs(c):
     src = make_source(c["seed"], c["S"])
     rir = make_rir(c["seed"], c["L"]) if c["L"] > 0 else None
@@ -76,6 +92,32 @@ def continuous_inputs(c):
     rir = make_rir(c["seed"], c["L"]).astype(np.float64)       # habitat-sim lists -> float64 (:419)
     last = make_rir(c["last_seed"], c["last_L"]).astype(np.float64) if "last_seed" in c else None
     return src, rir, last
+
+
+def reference_class_facts(ref):
+    """What ``patch_simulator`` meets in the reference's two simulator classes: every member name (with its kind), every
+    ``self.<name>`` their module mentions (attributes set by ``__init__`` / ``reconfigure``), and for the discrete class
+    the values its own properties return on the bare object ``ref_harness.make_discrete_sim`` builds."""
+    facts = {}
+    for key, mod in (("SoundSpacesSim", ref["simulator"]), ("ContinuousSoundSpacesSim", ref["continuous"])):
+        cls = getattr(mod, key)
+        members = {}
+        for n in dir(cls):
+            if not n.startswith("__"):
+                v = inspect.getattr_static(cls, n)
+                members[n] = "property" if isinstance(v, property) else "function" if inspect.isfunction(v) else "other"
+        with open(mod.__file__) as f:
+            self_attrs = sorted(set(re.findall(r"self\.(\w+)", f.read())))
+        facts[key] = {"members": members, "self_attributes": self_attrs}
+    root = os.path.join("rir", "root")
+    clip = np.zeros(16000, np.float32)
+    sims = {rot: rh.make_discrete_sim(ref, root, 16000, source_sounds={"telephone.wav": clip}, rotation_angle=rot)
+            for rot in (0, 90, 180, 270)}
+    assert all(s.current_source_sound is clip for s in sims.values())
+    facts["SoundSpacesSim"]["bare_object"] = {
+        "binaural_rir_dir_under_root": os.path.relpath(sims[0].binaural_rir_dir, root),
+        "azimuth_angle_by_rotation": {str(rot): int(s.azimuth_angle) for rot, s in sims.items()}}
+    return facts
 
 
 def main():
@@ -148,16 +190,38 @@ def main():
         out["singing/spec_reflect"] = sim.get_current_spectrogram_observation(
             ref["nav"].SpectrogramSensor.compute_spectrogram)
 
-    # keep the file small: waveforms at 44.1/48 kHz are stored as every 5th sample
-    packed = {}
+    c = AUDIO_INDEX_CASE
+    src, rir = make_source(c["seed"], c["S"]), make_rir(c["seed"], c["L"])
+    azimuth = -c["rotation_angle"] % 360
+    with tempfile.TemporaryDirectory() as d:
+        rh.write_rir(d, c["dataset"], c["scene"], azimuth, c["receiver"], c["source"], c["sr"], rir)
+        for idx in c["audio_indices"]:
+            sim = rh.make_discrete_sim(ref, d, c["sr"], dataset=c["dataset"], scene=c["scene"], receiver=c["receiver"],
+                                       source=c["source"], rotation_angle=c["rotation_angle"],
+                                       source_sounds={"telephone.wav": src}, audio_index=idx)
+            out[f"audio_index_{idx}/wave"] = sim.get_current_audiogoal_observation()
+            out[f"audio_index_{idx}/spec_reflect"] = sim.get_current_spectrogram_observation(
+                ref["nav"].SpectrogramSensor.compute_spectrogram)
+
+    # keep each file under 1 MB: waveforms go to a file of their own, most of them as every 5th sample
+    packed, waves = {}, {}
     for k, v in out.items():
-        if k.endswith("/wave") and v.shape[-1] > 16000:
-            packed[k + "_stride5"] = np.ascontiguousarray(v[:, ::5])
-        else:
+        if not k.endswith("/wave"):
             packed[k] = v
-    path = os.path.join(ROOT, "tests", "golden", "reference_golden.npz")
-    np.savez_compressed(path, **packed)
-    print("wrote", path, os.path.getsize(path), "bytes,", len(packed), "arrays")
+        elif k.startswith(tuple(CONTINUOUS_CASES)) or k in FULL_WAVES:
+            waves[k] = v
+        else:
+            waves[k + "_stride5"] = np.ascontiguousarray(v[:, ::5])
+    for name, arrays in (("reference_golden.npz", packed), ("reference_golden_waves.npz", waves)):
+        path = os.path.join(ROOT, "tests", "golden", name)
+        np.savez_compressed(path, **arrays)
+        print("wrote", path, os.path.getsize(path), "bytes,", len(arrays), "arrays")
+
+    path = os.path.join(ROOT, "tests", "golden", "reference_classes.json")
+    with open(path, "w") as f:
+        json.dump(reference_class_facts(ref), f, indent=1, sort_keys=True)
+        f.write("\n")
+    print("wrote", path)
 
     edge = {}
     ref = rh.load_reference("reflect")

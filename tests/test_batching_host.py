@@ -1,8 +1,9 @@
 """CPU tests of the host logic behind the per-env plugin surface (no CUDA: a stand-in renderer records the
 launches): the deferred-handle batcher and its ring, the ``batch_obs`` replacement, the scene-safe memo of
 ``VectorAudioObservations``, the RIR service (prefetch, misses, LRU compaction), the continuous simulator's
-wrap rule, and ``patch_simulator`` applied to the REAL reference classes."""
+wrap rule, and ``patch_simulator`` applied to classes with the REAL reference classes' members."""
 import gc
+import json
 import os
 import time
 
@@ -252,16 +253,26 @@ def test_continuous_wrap_only_in_steady_state_branch():
 
 
 # ---------------------------------------------------------------------------------- the real reference classes
-@pytest.mark.needs_reference
+def reference_stand_in(name):
+    """A class with every member name of the reference's simulator class ``name`` (recorded from the unmodified
+    reference by tests/golden/make_golden.py), each a placeholder of its kind, and the recorded facts."""
+    with open(os.path.join(os.path.dirname(__file__), "golden", "reference_classes.json")) as f:
+        facts = json.load(f)[name]
+
+    def placeholder(self, *a, **k):
+        raise AssertionError("reference member called")
+    ns = {n: property(placeholder) if kind == "property" else placeholder if kind == "function" else object()
+          for n, kind in facts["members"].items()}
+    return type("Patched" + name, (), ns), facts
+
+
 def test_patch_simulator_on_reference_classes():
-    """INTEGRATION.md advertises ``patch_simulator(SoundSpacesSim)``: apply it to the REAL classes (loaded unmodified
-    by oracle/ref_harness.py) with the renderer stubbed; exactly the three audio methods are replaced, everything
-    the replacements read exists on the reference object, and the patched object renders through the service."""
-    from oracle import ref_harness
-    ref = ref_harness.load_reference()
-    Sim = type("PatchedSoundSpacesSim", (ref["simulator"].SoundSpacesSim,), {})
-    CSim = type("PatchedContinuousSim", (ref["continuous"].ContinuousSoundSpacesSim,), {})
-    before = {n: getattr(Sim, n) for n in dir(ref["simulator"].SoundSpacesSim) if not n.startswith("__")}
+    """INTEGRATION.md advertises ``patch_simulator(SoundSpacesSim)``: apply it to classes with the REAL classes' members
+    with the renderer stubbed; exactly the three audio methods are replaced, everything the replacements read exists on
+    the reference object, and the patched object renders through the service."""
+    Sim, facts = reference_stand_in("SoundSpacesSim")
+    CSim, cfacts = reference_stand_in("ContinuousSoundSpacesSim")
+    before = {n: getattr(Sim, n) for n in facts["members"]}
     patch_simulator(Sim, deferred=True)
     patch_simulator(CSim, continuous=True)
     changed = sorted(n for n, v in before.items() if getattr(Sim, n) is not v)
@@ -269,20 +280,25 @@ def test_patch_simulator_on_reference_classes():
     added = sorted(n for n in dir(Sim) if n not in before and not n.startswith("__"))
     assert all(n.startswith(("_b200", "b200_")) or n == "get_current_audiogoal_device" for n in added), added
     # every attribute the patched methods read is provided by the reference class or set by its __init__/reconfigure
-    src = open(ref["simulator"].__file__).read()
     for name in DISCRETE_READS:
-        assert hasattr(ref["simulator"].SoundSpacesSim, name) or f"self.{name}" in src, name
-    csrc = open(ref["continuous"].__file__).read()
+        assert name in facts["members"] or name in facts["self_attributes"], name
     for name in CONTINUOUS_READS:
-        assert hasattr(ref["continuous"].ContinuousSoundSpacesSim, name) or f"self.{name}" in csrc, name
+        assert name in cfacts["members"] or name in cfacts["self_attributes"], name
 
-    # drive a patched REAL object (bare instance, App. D attributes) through the service with the renderer stubbed
+    # drive a patched object (bare instance, App. D attributes) through the service with the renderer stubbed; the
+    # properties the replacements read return what the reference's own properties returned on the same bare object
+    bare = facts["bare_object"]
+    Sim.binaural_rir_dir = property(lambda s: os.path.join(s.config.AUDIO.BINAURAL_RIR_DIR, bare["binaural_rir_dir_under_root"]))
+    Sim.azimuth_angle = property(lambda s: bare["azimuth_angle_by_rotation"][str(s._rotation_angle)])
+    Sim.current_source_sound = property(lambda s: s._source_sound_dict[s._current_sound])
     import tempfile
+    import types
+    from oracle import ref_harness
     sr = 16000
     with tempfile.TemporaryDirectory() as d:
         write_rir(d, "replica", "apartment_0", 0, 0, 1, sr, make_rir(3, 500))
+        ref = {"simulator": types.SimpleNamespace(SoundSpacesSim=Sim)}
         sim = ref_harness.make_discrete_sim(ref, d, sr, source_sounds={"telephone.wav": make_source(1, sr)})
-        sim.__class__ = Sim
         svc = make_service(sr)
         sim._b200_svc = svc
         sim.graph = None

@@ -2,6 +2,7 @@
 numpy model of the kernels' dataflow), the C-ABI library's exported symbols and struct layout,
 and the env sharding over a world_size-2 gloo group."""
 import ctypes
+import json
 import os
 import re
 import subprocess
@@ -273,11 +274,10 @@ def test_prepare_arrays_equals_prepare():
 
 # ---------------------------------------------------------------------------------- bench.py timed_region across ranks
 def _timed_region_worker(rank, world, port, tmp):
-    """Two gloo ranks whose local first measurement falls on different sides of the repeat threshold: the repeat count
-    (every repetition contains barriers) must still be the same on both, or the run deadlocks."""
+    """Two gloo ranks of different speed: each times exactly the K steps it was asked for, once, between barriers
+    (any extra region on one rank alone would leave the other waiting in a barrier)."""
     import time
     import types
-    import torch
     import torch.distributed as dist
     sys.path.insert(0, ROOT)
     import bench
@@ -293,26 +293,21 @@ def _timed_region_worker(rank, world, port, tmp):
             return (other.t - self.t) * 1e3
     fake_torch = types.SimpleNamespace(cuda=types.SimpleNamespace(Event=FakeEvent))
     dist.init_process_group("gloo", init_method=f"tcp://127.0.0.1:{port}", rank=rank, world_size=world)
-
-    def allmax(x):
-        t = torch.tensor([x], dtype=torch.float64)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t.item())
-    bench.MIN_REGION_S = 0.02
     calls = []
 
     def step(i):
         calls.append(i)
-        time.sleep(0.0015 if rank == 0 else 0.0004)          # rank 0: 15 ms per region, rank 1: 4 ms: different local repeat counts
-    ms, reps, total = bench.timed_region(step, 10, dist.barrier, fake_torch, allmax=allmax)
-    open(os.path.join(tmp, f"reps{rank}"), "w").write(str(reps))
+        time.sleep(0.0015 if rank == 0 else 0.0004)          # rank 0: 15 ms per region, rank 1: 4 ms
+    ms = bench.timed_region(step, 10, dist.barrier, fake_torch)
+    open(os.path.join(tmp, f"region{rank}"), "w").write(json.dumps({"calls": calls, "ms": ms}))
     dist.barrier()
     dist.destroy_process_group()
 
 
-def test_bench_timed_region_repeat_count_is_rank_consistent(tmp_path):
+def test_bench_timed_region_times_exactly_k_steps_on_every_rank(tmp_path):
     import torch.multiprocessing as mp
     port = 29300 + os.getpid() % 300
     mp.spawn(_timed_region_worker, args=(2, port, str(tmp_path)), nprocs=2, join=True)
-    r0, r1 = (int(open(tmp_path / f"reps{k}").read()) for k in (0, 1))
-    assert r0 == r1 and r0 >= 3
+    r0, r1 = (json.loads(open(tmp_path / f"region{k}").read()) for k in (0, 1))
+    assert r0["calls"] == r1["calls"] == list(range(10))
+    assert r0["ms"] >= 15.0 and r1["ms"] >= 4.0
